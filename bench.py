@@ -27,6 +27,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 LOG_DEG = 20
 CURVE = "bls12_381"
@@ -44,6 +45,9 @@ def parse():
     ap.add_argument("--no-sharded", action="store_true", help="skip the sharded MSM / cfg5 / NTT sub-record")
     ap.add_argument("--sharded-log-n", type=int, default=22)
     ap.add_argument("--cfg5-polys", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the commitment and witness of the last timed step to DIR/<name>.npy "
+                         "(float64; each 64-bit Montgomery limb of x||y as two 32-bit words, low word first)")
     return ap.parse_args()
 
 
@@ -184,6 +188,16 @@ def cpu_reference_run(args, log_deg, steps, warmup, budget_s):
             "ms_per_step": t * 1e3, "msm_scalar_mults_per_s": 2 * n_full / t}
 
 
+def dump_outputs(out_dir, c, ci, w, wi):
+    """the arrays the batch call returns for one polynomial, exactly: 64-bit limbs split into 32-bit words fit float64"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    words = lambda xy: np.ascontiguousarray(xy, dtype=np.uint64).view(np.uint32).astype(np.float64)
+    for name, a in (("commitment_xy", words(c)), ("commitment_inf", np.float64([ci])),
+                    ("witness_xy", words(w)), ("witness_inf", np.float64([wi]))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     args = parse()
     rank = int(os.environ.get("RANK", "0"))
@@ -266,7 +280,7 @@ def main():
         e0.record()
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        fn(k)
+        res = fn(k)
         torch.cuda.synchronize()
         wall_ms = (time.perf_counter() - t0) * 1e3
         e1.record()
@@ -276,18 +290,20 @@ def main():
             t = torch.tensor([ms], device="cuda")
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms
+        return ms, res
 
     sampler = ClockSampler(local_rank)
     sampler.start()                      # started before the warm-up so nvidia-smi is already streaming samples
     run_dev(max(warmup, 3))
     sampler.mark()
     l0 = eng.launch_count()
-    ms_dev = timed(run_dev, steps)
+    ms_dev, (c, ci, w, wi) = timed(run_dev, steps)
     launches = eng.launch_count() - l0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, c[-1], ci[-1], w[-1], wi[-1])
     run_host(max(warmup, 3))
-    ms_host = timed(run_host, steps)
+    ms_host, _ = timed(run_host, steps)
     # single-call latency (one polynomial per call: what a serial Rust caller of commit-then-open sees)
     eng.kzg_commit_open(srs, dev_polys[0].data_ptr(), z, n=n, flags=pc.DEVICE_PTRS)
     torch.cuda.synchronize()

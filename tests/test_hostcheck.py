@@ -288,17 +288,20 @@ def test_kzg_commit_open_fused(eng, pc):
     with pytest.raises(pc.PcgpuError) as ei:
         eng.kzg_commit_open(pg, util.rand_fr(cname, n + 1, seed=404, mont=True), z)
     assert ei.value.code == -6
-    # "device" pointers (host pointers under emulation): the trailing zeros must be trimmed on the device side as well
+    # device-resident coefficients (the engine's own buffers: host memory under emulation): the trailing zeros must be trimmed
+    # on the device side as well
     for p, e in zip(polys, exp):
-        (c, ci), (w, wi) = eng.kzg_commit_open(pg, p.ctypes.data, z, n=p.shape[0], flags=pc.DEVICE_PTRS)
+        d = eng.buffer(p.shape[0])
+        d.write(p)
+        (c, ci), (w, wi) = eng.kzg_commit_open(pg, d.ptr(), z, n=p.shape[0], flags=pc.DEVICE_PTRS)
         assert (c == e[0]).all() and ci == e[1] and (w == e[2]).all() and wi == e[3]
-        got = eng.kzg_commit(pg, p.ctypes.data, n=p.shape[0], flags=pc.DEVICE_PTRS)
+        got = eng.kzg_commit(pg, d.ptr(), n=p.shape[0], flags=pc.DEVICE_PTRS)
         assert (got[0] == e[0]).all() and got[1] == e[1]
-    padded = np.zeros((n + 50, 4), dtype=np.uint64)
-    padded[:n] = polys[0]
-    got = eng.kzg_commit(pg, padded.ctypes.data, n=n + 50, flags=pc.DEVICE_PTRS)   # zero-padded beyond the SRS length: no E_DEGREE
+    d = eng.buffer(n + 50)                                                   # zero-filled
+    d.write(polys[0])
+    got = eng.kzg_commit(pg, d.ptr(), n=n + 50, flags=pc.DEVICE_PTRS)   # zero-padded beyond the SRS length: no E_DEGREE
     assert (got[0] == exp[0][0]).all()
-    got = eng.kzg_open(pg, padded.ctypes.data, z, n=n + 50, flags=pc.DEVICE_PTRS)
+    got = eng.kzg_open(pg, d.ptr(), z, n=n + 50, flags=pc.DEVICE_PTRS)
     assert (got[0] == exp[0][2]).all()
 
 
