@@ -29,10 +29,15 @@ def eng(gpu_engine):
     return gpu_engine
 
 
+def gpu_srs_beta(cname, seed=1):
+    """the trapdoor beta (Montgomery form) of gpu_srs(..., seed): test_degenerate_srs checks commitments against p(beta) * G"""
+    return util.rand_fr(cname, 1, 1000 + seed, mont=True)[0]
+
+
 def gpu_srs(eng, cname, n, seed=1):
     """powers_of_g = beta^i * G built ON THE DEVICE (pcgpu_g1_fixed_base_mul), spot-checked against the oracle."""
     C = pyref.Curve(cname)
-    beta = util.rand_fr(cname, 1, 1000 + seed, mont=True)[0]
+    beta = gpu_srs_beta(cname, seed)
     pows = orc.fr_powers_canonical(C.id, beta, n)
     xy = eng.fixed_base_mul(C.id, orc.g1_generator(C.id), pows)
     idx = np.unique(np.concatenate([[0, 1, n - 1], util.rng(seed).integers(0, n, size=12)]))
@@ -142,10 +147,18 @@ def test_cfg2_fused_commit_open(eng, pc, big):
     assert rc == 0 and rc2 == 0
     (c, ci), (w, wi) = eng.kzg_commit_open(big["srs"], big["coeffs"], z)
     assert (c == exy).all() and ci == einf and (w == wxy).all() and wi == winf
-    d = torch.from_numpy(big["coeffs"].view(np.int64)).cuda()
-    cb, cib, wb, wib = eng.kzg_commit_open_batch(big["srs"], [(d.data_ptr(), n)] * 3, z, flags=pc.DEVICE_PTRS)
-    for i in range(3):
-        assert (cb[i] == exy).all() and cib[i] == einf and (wb[i] == wxy).all() and wib[i] == winf
+    # three distinct polynomials in flight: a result in the wrong slot or cross-talk between the ways shows.  The two new ones are
+    # checked against the trapdoor formulas (p(beta) * G, test_degenerate_srs), the first against the oracle above.
+    from tests.test_degenerate_srs import ref_commit, ref_witness
+    beta = C.fr_from_limbs(gpu_srs_beta("bls12_381", 20), True)[0]
+    zi = C.fr_from_limbs(z, True)[0]
+    others = [util.rand_fr_fast("bls12_381", n, seed=75), util.rand_fr_fast("bls12_381", n // 2 + 3, seed=76)]
+    others[0][-4321:] = 0
+    exp = [((exy, einf), (wxy, winf))] + [(ref_commit(C, p, beta), ref_witness(C, p, beta, zi)) for p in others]
+    ds = [torch.from_numpy(p.view(np.int64)).cuda() for p in [big["coeffs"]] + others]
+    cb, cib, wb, wib = eng.kzg_commit_open_batch(big["srs"], [(d.data_ptr(), d.shape[0]) for d in ds], z, flags=pc.DEVICE_PTRS)
+    for i, ((ec, eci), (ew, ewi)) in enumerate(exp):
+        assert cib[i] == eci and wib[i] == ewi and (cb[i] == ec).all() and (wb[i] == ew).all(), i
 
 
 def test_cfg2_properties(eng, pc, big):
